@@ -135,6 +135,21 @@ def measured_peaks():
     return {"hbm_gbs": 6650.0}, "fallback"
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each array as dirname/<name>.npy, so that two builds can be compared output for output on the same
+    seeded workload.  Every workload's film (at most 1920x1080) fits the limit whole, so nothing is sampled."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError("outputs of %d bytes exceed the %d-byte dump limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def write_reference_scene(scenes, arr, wl, spp, tmp):
     n_tris, mats, xres, yres, _, depth, n_lights, _ = wl
     return scenes.write_pbrt(tmp, "bench", arr, xres, yres, spp, max_depth=depth, strategy="uniform", **getattr(arr, "bench_integrator", {}))
@@ -187,7 +202,11 @@ def main():
                     help="a key of tests/golden/filter_tables.json (gaussian, mitchell, sinc ...); default: box filter")
     ap.add_argument("--bvh", default="host", choices=["host", "gpu"],
                     help="acceleration structure builder: host SAH (default) or the on-device builder")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the film of the last timed step as DIR/image_rgb.npy and DIR/film_raw.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, local_rank, world = rank_env()
     wl = WORKLOADS[args.workload]
     n_tris, mats, xres, yres, spp, depth, n_lights, desc = wl
@@ -390,6 +409,9 @@ def main():
 
     ms, rays, samples, st, clocks, _ = timed(False, args.steps, args.warmup)
     rank_ms = list(timed.rank_ms)
+    if args.dump_outputs and rank == 0:
+        # read before the end-to-end leg renders into the same film; on rank 0 it holds every rank's reduced sums
+        dump_outputs(args.dump_outputs, {"image_rgb": render.read_rgb(), "film_raw": render.read_raw()})
     e2e_steps = args.e2e_steps if args.e2e_steps else min(args.steps, 5)
     ms_e, rays_e, samples_e, st_e, _, h2d = timed(True, e2e_steps, 1)
     # one more end-to-end step with events between its three parts (reported, not part of any timed figure)
